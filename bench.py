@@ -3,6 +3,7 @@
     python bench.py --gpus 1 --steps 3 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference algorithm's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one separate() over a batch of B synthetic clips per GPU (weak scaling): DAC-VAE encode,
 conditioning, 32 DiT evaluations (midpoint ODE), DAC-VAE decode of target+residual, and — for N>1 — the
@@ -247,6 +248,39 @@ SAMPLE_DESC = ("1 clip (10 s @ 48 kHz) through the oracle port on the host cores
                "midpoint steps (2 DiT evaluations, x16) + DAC-VAE decode of target+residual; fp32 torch")
 
 
+DUMP_BYTES = 60_000_000       # --dump-outputs writes at most this much in all (under 64 MB with the .npy headers)
+
+
+def step_outputs(out):
+    """What a caller of the timed step receives, as [rows, ...] tensors: separate()'s SeparationResult at N = 1, the
+    all-gathered [N*B, 2, samples] target/residual waveforms at N > 1."""
+    if torch.is_tensor(out):
+        return {"target": out[:, 0], "residual": out[:, 1]}
+    return {"target": torch.stack(out.target), "residual": torch.stack(out.residual), "noise": out.noise}
+
+
+def sample_outputs(arrays):
+    """float32 host copies of `arrays`.  One larger than its equal share of DUMP_BYTES keeps a fixed seeded sample of its
+    columns (the same columns in every row), so that two runs with the same arguments can be compared value for value."""
+    share = DUMP_BYTES // len(arrays)
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().float().reshape(a.shape[0], -1)
+        cols = max(1, share // (4 * a.shape[0]))
+        if cols < a.shape[1]:
+            keep = torch.randperm(a.shape[1], generator=torch.Generator().manual_seed(0))[:cols].sort().values
+            a = a[:, keep.to(a.device)]
+        out[name] = a.cpu()
+    return out
+
+
+def write_outputs(arrays, out_dir):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+
+
 def run_reference(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -417,11 +451,19 @@ def run_gpu(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms)
 
+    last = {}
+
+    def step_value():
+        last.clear()                            # the previous step's result is freed before this step runs
+        last["out"] = step_resident(batch_gpu, noise_gpu)
+
     sampler = ClockSampler(local) if rank == 0 else None
     # ---- value: inputs resident in HBM (the ODE solve replays as one CUDA graph) ----
     eng.launch_count(reset=True)
-    ms_val = timed(lambda: step_resident(batch_gpu, noise_gpu), args.steps)
+    ms_val = timed(step_value, args.steps)
     launches = eng.launch_count(reset=True)
+    dumped = sample_outputs(step_outputs(last["out"])) if args.dump_outputs and rank == 0 else None
+    last.clear()
     # ---- the same K steps again with one CUDA event in front of every launch: live per-kernel times ----
     eng.profile(True)
     ms_prof = timed(lambda: step_resident(batch_gpu, noise_gpu), args.steps)
@@ -438,6 +480,8 @@ def run_gpu(args):
             import torch.distributed as dist
             dist.destroy_process_group()
         return
+    if dumped is not None:
+        write_outputs(dumped, args.dump_outputs)
     peaks = _peaks()
     clips_total = world * B * args.steps
     value = clips_total / (ms_val / 1e3)
@@ -554,7 +598,12 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--gather", default="overlap", choices=["overlap", "after"],
                     help="N>1: all-gather each decoded chunk under the next chunk's decode, or once after the decode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32; arrays above their share of "
+                         f"{DUMP_BYTES // 10**6} MB keep a fixed seeded sample of columns)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -20,6 +20,7 @@ from __future__ import annotations
 import os
 import sys
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,9 +32,48 @@ from sam_audio_b200.config import stand_in_config  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
+# Every fixture stays under 1 MB: seeded random inputs are stored as (shape, seed) plus their first HEAD values, which
+# the loaders below check after regenerating them, and separate_tiny.pt keeps one waveform sample in WAV_KEEP.
+HEAD = 64
+WAV_KEEP = 4
+VIDEO_SEED = 8
+
 
 def rel_l2(a, b):
     return float((a.double() - b.double()).norm() / b.double().norm().clamp_min(1e-30))
+
+
+def wav_positions(n: int) -> torch.Tensor:
+    """The positions of an n-sample waveform that separate_tiny.pt stores: a fixed pseudo-random 1/WAV_KEEP of them,
+    sorted (numpy's legacy RandomState stream does not change between versions)."""
+    return torch.from_numpy(np.sort(np.random.RandomState(n).choice(n, n // WAV_KEEP, replace=False)))
+
+
+def _seeded_video(shape, seed):
+    return torch.randn(shape, generator=torch.Generator().manual_seed(seed))
+
+
+def _check_head(t, head):
+    assert torch.equal(t.flatten()[:HEAD], head), "the seeded generator no longer reproduces this golden input"
+
+
+def load_samaudio_forward(golden_dir):
+    """samaudio_forward_tiny.pt with its video input regenerated from the stored seed."""
+    g = torch.load(os.path.join(golden_dir, "samaudio_forward_tiny.pt"))
+    g["video"] = _seeded_video(g["video_shape"], g["video_seed"])
+    _check_head(g["video"], g["video_head"])
+    return g
+
+
+def load_separate(golden_dir):
+    """separate_tiny.pt with each result's noise regenerated from the stored seed.  "target" / "residual" hold each
+    clip's waveform at wav_positions(n) only; the full lengths n are in "wav_lens"."""
+    g = torch.load(os.path.join(golden_dir, "separate_tiny.pt"))
+    for r in g["results"].values():
+        bc, t, ch = r["noise_shape"]
+        r["noise"] = synthetic.synthetic_noise(bc, t, ch, seed=r["noise_seed"])
+        _check_head(r["noise"], r["noise_head"])
+    return g
 
 
 class _RestatedCodec(torch.nn.Module):
@@ -176,7 +216,7 @@ def main():
     feats = torch.randn(B, T, 128, generator=g)
     feats = torch.cat([feats, feats], 2)
     text = torch.randn(B, L, 768, generator=g)
-    video = torch.randn(B, 1024, T, generator=g)
+    video = _seeded_video((B, 1024, T), VIDEO_SEED)
     anc = [[["+", 0.1, 0.5]], [["-", 0.0, 0.2], ["+", 0.1, 0.9]], []]
     ids, al = restate.process_anchors(anc, pad_mask, 1920, 48000)
     outs = {}
@@ -199,7 +239,8 @@ def main():
         print(f"SAMAudio.forward[{tag}] restatement vs reference: rel_l2={e:.3e}")
         assert e < 2e-5, e
         outs[tag] = r
-    torch.save(dict(noisy=noisy, feats=feats, text=text, video=video, time=time, text_mask=mem_mask,
+    torch.save(dict(noisy=noisy, feats=feats, text=text, video_shape=tuple(video.shape), video_seed=VIDEO_SEED,
+                    video_head=video.flatten()[:HEAD].clone(), time=time, text_mask=mem_mask,
                     anchor_ids=ids, anchor_alignment=al, pad_mask=pad_mask, out=outs),
                os.path.join(GOLDEN, "samaudio_forward_tiny.pt"))
 
@@ -229,10 +270,15 @@ def main():
     auds2 = [synthetic.synthetic_clip(i, n) for i, n in enumerate(lens2)]
     desc2 = synthetic.synthetic_descriptions(2)
     sep = {}
+
+    def stored(r, noise, seed, **extra):
+        return dict(target=[t[wav_positions(t.numel())].clone() for t in r.target],
+                    residual=[t[wav_positions(t.numel())].clone() for t in r.residual], noise_shape=tuple(noise.shape),
+                    noise_seed=seed, noise_head=noise.flatten()[:HEAD].clone(), **extra)
     for cand in (1, 2, 8):
         batch = proc(descriptions=desc2, audios=auds2)
         Tn = int(batch.sizes.max())
-        noise = synthetic.synthetic_noise(2 * cand, Tn)
+        noise = synthetic.synthetic_noise(2 * cand, Tn, seed=4321)
         r = model.separate(batch, noise=noise, reranking_candidates=cand)
         tf, tm = synthetic.synthetic_text_features(desc2)
         tgt, res, lat = restate.separate(sd, cfg, batch.audios, batch.audio_pad_mask, batch.sizes, tf, tm,
@@ -244,8 +290,7 @@ def main():
             assert e < 1e-4, e
         print(f"separate(candidates={cand}) restatement vs reference pipeline: ok "
               f"(lens {[t.numel() for t in r.target]})")
-        sep[cand] = dict(target=[t.clone() for t in r.target], residual=[t.clone() for t in r.residual],
-                         latent=lat, noise=noise)
+        sep[cand] = stored(r, noise, 4321, latent=lat)
     # candidate selection through an attached text ranker (model.py:316-328): a stand-in with fixed scores — the
     # call-site logic (argument shapes, argmax, which candidate's waveforms are returned) is the reference's
     class _FixedRanker(torch.nn.Module):
@@ -260,9 +305,9 @@ def main():
     noise = synthetic.synthetic_noise(2 * 3, int(batch.sizes.max()), seed=777)
     r = model.separate(batch, noise=noise, reranking_candidates=3)
     model.text_ranker = None
-    sep["ranked3"] = dict(target=[t.clone() for t in r.target], residual=[t.clone() for t in r.residual], noise=noise,
-                          scores=_FixedRanker.SCORES.clone())
-    torch.save(dict(lens=lens2, results=sep), os.path.join(GOLDEN, "separate_tiny.pt"))
+    sep["ranked3"] = stored(r, noise, 777, scores=_FixedRanker.SCORES.clone())
+    torch.save(dict(lens=lens2, wav_lens=[t.numel() for t in r.target], results=sep),
+               os.path.join(GOLDEN, "separate_tiny.pt"))
     for f in sorted(os.listdir(GOLDEN)):
         print(f, os.path.getsize(os.path.join(GOLDEN, f)))
 

@@ -10,12 +10,11 @@ Tolerances (bf16 tensor-core operands, fp32 accumulation and fp32 residual strea
   * separate() waveforms vs reference (32 evaluations compound) ............ SNR >= 30 dB
   * integer outputs (sizes, lengths, masks, anchors) ....................... bit-exact
 """
-import os
-
 import pytest
 import torch
 
 from _util import rel_l2, snr_db
+from oracle.make_golden import load_samaudio_forward, load_separate, wav_positions
 
 pytestmark = pytest.mark.gpu
 
@@ -144,7 +143,7 @@ def test_long_sequence_uses_streaming_attention(tiny_model):
 def test_dit_evaluation_vs_reference_golden(tiny_model, golden_dir):
     """SAMAudio.forward (ragged pad mask, text mask, anchors, with and without video) vs the reference's
     own SAMAudio.forward output (tests/golden/samaudio_forward_tiny.pt)."""
-    g = torch.load(os.path.join(golden_dir, "samaudio_forward_tiny.pt"))
+    g = load_samaudio_forward(golden_dir)
     for tag, vid in (("video", g["video"]), ("novideo", torch.zeros_like(g["video"]))):
         out = tiny_model.forward(g["noisy"].cuda(), g["feats"].cuda(), g["text"].cuda(), g["time"].cuda(),
                                  masked_video_features=vid.cuda(),
@@ -156,7 +155,7 @@ def test_dit_evaluation_vs_reference_golden(tiny_model, golden_dir):
 def test_dit_evaluation_none_arguments_vs_reference_golden(tiny_model, golden_dir):
     """The `None` cases of SAMAudio.forward mean what they mean in the reference: no video term (align.py:41-42),
     no anchor term (model.py:57-58), time-only memory (model.py:170-172) — golden = the reference's own output."""
-    g = torch.load(os.path.join(golden_dir, "samaudio_forward_tiny.pt"))
+    g = load_samaudio_forward(golden_dir)
     out = tiny_model.forward(g["noisy"].cuda(), g["feats"].cuda(), g["text"].cuda(), g["time"].cuda(),
                              text_mask=g["text_mask"].cuda(), audio_pad_mask=g["pad_mask"].cuda())
     assert rel_l2(out.cpu(), g["out"]["none_video_anchors"]) < 2e-2
@@ -290,16 +289,17 @@ def test_separate_vs_reference_golden(tiny_model, golden_dir, cand):
     conditioning inside the engine instead of the reference's expand/reshape copies, model.py:193-203)."""
     from sam_audio_b200 import SAMAudioProcessor
     from sam_audio_b200.synthetic import synthetic_clip, synthetic_descriptions
-    g = torch.load(os.path.join(golden_dir, "separate_tiny.pt"))
+    g = load_separate(golden_dir)
     proc = SAMAudioProcessor(1920, 48000)
     auds = [synthetic_clip(i, n) for i, n in enumerate(g["lens"])]
     batch = proc(descriptions=synthetic_descriptions(2), audios=auds).to("cuda")
     r = g["results"][cand]
     out = tiny_model.separate(batch, noise=r["noise"].cuda(), reranking_candidates=cand)
     assert torch.equal(out.noise.cpu(), r["noise"])
-    for ours, ref in zip(list(out.target) + list(out.residual), list(r["target"]) + list(r["residual"])):
-        assert ours.shape == ref.shape                      # lengths = sizes*1920, bit-exact
-        assert snr_db(ours.cpu(), ref) > 30.0
+    for ours, ref, n in zip(list(out.target) + list(out.residual), list(r["target"]) + list(r["residual"]),
+                            g["wav_lens"] * 2):
+        assert ours.shape == (n,)                           # lengths = sizes*1920, bit-exact
+        assert snr_db(ours.cpu()[wav_positions(n)], ref) > 30.0
     # every candidate's latent (not only the returned candidate 0) against the reference pipeline's ODE state
     assert rel_l2(tiny_model._last_latent.cpu(), r["latent"]) < 2e-2
 
@@ -327,7 +327,7 @@ def test_candidate_selection_through_attached_rankers_vs_reference_golden(tiny_m
     from sam_audio_b200 import SAMAudioProcessor
     from sam_audio_b200.ranking import EnsembleRanker
     from sam_audio_b200.synthetic import synthetic_clip, synthetic_descriptions
-    g = torch.load(os.path.join(golden_dir, "separate_tiny.pt"))
+    g = load_separate(golden_dir)
     r = g["results"]["ranked3"]
     proc = SAMAudioProcessor(1920, 48000)
     auds = [synthetic_clip(i, n) for i, n in enumerate(g["lens"])]
@@ -348,12 +348,15 @@ def test_candidate_selection_through_attached_rankers_vs_reference_golden(tiny_m
     # reference builds it (model.py:317-320): clip 0 is the longest, so its mixture is shorter than the hop-padded output
     assert seen["n"] == 2 and seen["cand"] == 3 and seen["sr"] == 48000
     assert seen["inp"][0] == 3 and seen["inp"][1] == g["lens"][0] <= seen["ext"][1]
-    for ours, ref in zip(list(out.target) + list(out.residual), list(r["target"]) + list(r["residual"])):
-        assert ours.shape == ref.shape and snr_db(ours.cpu(), ref) > 30.0
+    for ours, ref, n in zip(list(out.target) + list(out.residual), list(r["target"]) + list(r["residual"]),
+                            g["wav_lens"] * 2):
+        assert ours.shape == (n,) and snr_db(ours.cpu()[wav_positions(n)], ref) > 30.0
     # without the ranker candidate 0 is returned: clip 0 differs from the ranked result, clip 1 (winner 0) does not
     plain = tiny_model.separate(proc(descriptions=synthetic_descriptions(2), audios=auds).to("cuda"),
                                 noise=r["noise"].cuda(), reranking_candidates=3)
-    assert snr_db(plain.target[0].cpu(), r["target"][0]) < 20.0 and torch.equal(plain.target[1], out.target[1])
+    n0 = g["wav_lens"][0]
+    assert snr_db(plain.target[0].cpu()[wav_positions(n0)], r["target"][0]) < 20.0
+    assert torch.equal(plain.target[1], out.target[1])
 
 
 def test_separate_with_anchors_vs_oracle(tiny_model, tiny_cfg, tiny_sd):
@@ -473,7 +476,7 @@ def test_exact_softmax_fallback_and_many_anchor_ids(tiny_cfg, tiny_sd, golden_di
     m = m.eval().cuda()
     m._ensure_engine()                                     # the env is read when the weights are finalised
     monkeypatch.delenv("SAB_ATTN_EXACT")
-    g = torch.load(os.path.join(golden_dir, "samaudio_forward_tiny.pt"))
+    g = load_samaudio_forward(golden_dir)
     out = m.forward(g["noisy"].cuda(), g["feats"].cuda(), g["text"].cuda(), g["time"].cuda(),
                     masked_video_features=g["video"].cuda(), text_mask=g["text_mask"].cuda(),
                     anchor_ids=g["anchor_ids"].cuda(), anchor_alignment=g["anchor_alignment"].cuda(),

@@ -205,3 +205,32 @@ def test_bench_parity_gate_logic():
     assert not bench.parity_gate(bad, cpu)["ok"]
     bad = dict(near, velocity=-cpu["velocity"])
     assert not bench.parity_gate(bad, cpu)["ok"]
+
+
+def test_bench_output_dump_is_bounded_and_repeatable(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files within the byte budget; an array over its share keeps the same
+    seeded sample of columns in every row and in every run; small arrays are written whole."""
+    import numpy as np
+    import bench
+    from sam_audio_b200.model import SeparationResult
+    monkeypatch.setattr(bench, "DUMP_BYTES", 60_000)
+    B, S = 4, 48_000
+    wav = torch.arange(B * S, dtype=torch.float32).view(B, S)          # value = row * S + column
+    res = SeparationResult(target=list(wav), residual=list(-wav), noise=torch.randn(B, 5, 8).double())
+    for run in ("a", "b"):
+        bench.write_outputs(bench.sample_outputs(bench.step_outputs(res)), str(tmp_path / run))
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["noise.npy", "residual.npy", "target.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 60_000 + 3 * 128
+    a = {f: np.load(tmp_path / "a" / f) for f in files}
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / f)) for f, v in a.items())
+    t = a["target.npy"]
+    cols = t[0]
+    assert t.shape == (B, 20_000 // (4 * B)) and (np.diff(cols) > 0).all()
+    assert np.array_equal(t, cols[None] + S * np.arange(B, dtype=np.float32)[:, None])
+    assert np.array_equal(a["residual.npy"], -t)
+    assert np.array_equal(a["noise.npy"], res.noise.float().view(B, -1).numpy())
+    g = bench.sample_outputs(bench.step_outputs(torch.stack([wav, -wav], 1)))    # the N > 1 form: [N*B, 2, samples]
+    assert sorted(g) == ["residual", "target"] and torch.equal(g["residual"], -g["target"])
+    assert g["target"].shape == (B, 30_000 // (4 * B))

@@ -5,6 +5,7 @@ import os
 import torch
 
 from oracle import restate
+from oracle.make_golden import load_samaudio_forward, load_separate, wav_positions
 from sam_audio_b200 import synthetic
 from _util import rel_l2
 
@@ -19,7 +20,7 @@ def test_dit_forward_matches_reference_golden(golden_dir, tiny_cfg, tiny_sd):
 
 
 def test_samaudio_forward_matches_reference_golden(golden_dir, tiny_cfg, tiny_sd):
-    g = torch.load(os.path.join(golden_dir, "samaudio_forward_tiny.pt"))
+    g = load_samaudio_forward(golden_dir)
     for tag, vid in (("video", g["video"]), ("novideo", torch.zeros_like(g["video"]))):
         out = restate.samaudio_forward(tiny_sd, tiny_cfg, g["noisy"], g["feats"], g["text"], g["time"], vid,
                                        g["text_mask"], g["anchor_ids"], g["anchor_alignment"], g["pad_mask"])
@@ -77,7 +78,7 @@ def test_other_fixed_grid_solvers_orders_of_accuracy():
 
 def test_separate_control_flow_matches_reference_golden(golden_dir, tiny_cfg, tiny_sd):
     """encode -> 32 evaluations -> decode -> unbatch, candidates 1 and 8 (reference pipeline output)."""
-    g = torch.load(os.path.join(golden_dir, "separate_tiny.pt"))
+    g = load_separate(golden_dir)
     auds = [synthetic.synthetic_clip(i, n) for i, n in enumerate(g["lens"])]
     aud, ws = restate.batch_audio(auds)
     sizes = restate.wav_to_feature_idx(ws, 1920)
@@ -89,13 +90,13 @@ def test_separate_control_flow_matches_reference_golden(golden_dir, tiny_cfg, ti
         tgt, res, lat = restate.separate(tiny_sd, tiny_cfg, aud, mask, sizes, tf, tm, ids, al, r["noise"],
                                          candidates=cand, return_latent=True)
         assert lat.shape[0] == 2 * cand and rel_l2(lat, r["latent"]) < 1e-4
-        for a, b in zip(tgt + res, list(r["target"]) + list(r["residual"])):
-            assert a.shape == b.shape and rel_l2(a, b) < 1e-4
+        for a, b, n in zip(tgt + res, list(r["target"]) + list(r["residual"]), g["wav_lens"] * 2):
+            assert a.shape == (n,) and rel_l2(a[wav_positions(n)], b) < 1e-4
 
 
 def test_ranked_candidate_selection_matches_reference_golden(golden_dir, tiny_cfg, tiny_sd):
     """model.py:306-330 with an attached (stand-in, fixed-score) text ranker: arg-max candidate per clip."""
-    g = torch.load(os.path.join(golden_dir, "separate_tiny.pt"))
+    g = load_separate(golden_dir)
     r = g["results"]["ranked3"]
     auds = [synthetic.synthetic_clip(i, n) for i, n in enumerate(g["lens"])]
     aud, ws = restate.batch_audio(auds)
@@ -106,8 +107,8 @@ def test_ranked_candidate_selection_matches_reference_golden(golden_dir, tiny_cf
     tgt, res = restate.separate(tiny_sd, tiny_cfg, aud, mask, sizes, tf, tm, ids, al, r["noise"], candidates=3,
                                 ranker_scores=r["scores"])
     assert r["scores"].argmax(1).tolist() == [1, 0]
-    for a, b in zip(tgt + res, list(r["target"]) + list(r["residual"])):
-        assert a.shape == b.shape and rel_l2(a, b) < 1e-4
+    for a, b, n in zip(tgt + res, list(r["target"]) + list(r["residual"]), g["wav_lens"] * 2):
+        assert a.shape == (n,) and rel_l2(a[wav_positions(n)], b) < 1e-4
 
 
 def test_codec_shapes_and_hop(tiny_cfg, tiny_sd):
